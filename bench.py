@@ -2,6 +2,7 @@
 """bench.py — headline benchmark of the partitioned-convolution hot path (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload metric|ir120|...]
+                  [--dump-outputs DIR]
 
 Metric: M stereo frames / s ("Msamples/sec stereo conv @ IR=10s/48kHz block=512"): two
 independent mono convolutions (LL, RR — src/dsp/StereoConvolver.cpp:35-36) with their own
@@ -33,6 +34,11 @@ at every N ("strong" scaling).
                    ranks with the fused slot exchange over NVLink (north_star's multi-GPU case), every N.
 * cpu_baseline     the reference's own CPU code (oracle/_ref, unmodified sources) on this host's cores,
                    one pinned thread per core, instance memory first-touched by its own thread.
+
+--dump-outputs DIR writes the output the last timed step returned to its caller (the device array y[c][t] of the
+headline workload) as DIR/y.npy, float32, shape (channels, blocks, block): every block when the output fits in
+DUMP_BYTES, else the blocks of dump_blocks() (a fixed seeded sample with the first and the last block).  Inputs and
+IRs are seeded, so two builds run with the same arguments can be compared output for output.
 
 N > 1 (torchrun, one rank per GPU):
   metric shape (10 s IR, batch >> IR): TIME-SLICE sharding — every GPU holds the whole 7.7 MB convolver and
@@ -77,6 +83,7 @@ WORKLOADS = {
 # per-call fixed costs of a slice (history upload + transforms, pipeline fill of the PCIe path) stay small at N = 8
 T_METRIC = 112608
 T_IR120 = 7104
+DUMP_BYTES = 32 << 20          # --dump-outputs: at most this much of the step output (the metric's is 461 MB)
 
 
 def measured_peaks():
@@ -102,6 +109,16 @@ def measured_bf16_peaks():
 def algorithmic_bytes_per_channel_block(P: int, block: int) -> int:
     K = block + 1
     return 16 * P * K + 8 * K + 16 * block
+
+
+def dump_blocks(T: int, C: int, block: int) -> np.ndarray:
+    """Block indices of the step output --dump-outputs writes: all T blocks when they fit in DUMP_BYTES, else a fixed
+    seeded sample of that size that includes the first and the last block (sorted)."""
+    S = DUMP_BYTES // (C * block * 4)
+    if T <= S:
+        return np.arange(T)
+    mid = np.random.default_rng(T).choice(np.arange(1, T - 1), S - 2, replace=False)
+    return np.sort(np.concatenate([[0, T - 1], mid]))
 
 
 def slice_plan(T: int, P: int, rank: int, count: int):
@@ -345,8 +362,15 @@ def main():
     ap.add_argument("--mgpu", default="p2p", choices=["p2p", "nccl"], help="partition-range shards (120 s IR): exchange path")
     ap.add_argument("--metric-shards", dest="metric_shards", default="time", choices=["time", "partition"],
                     help="N > 1, metric shape: time-slice sharding (default) or partition-range shards")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", default=None, metavar="DIR",
+                    help="write the output of the last timed step as DIR/y.npy (float32, seeded sample of at most "
+                         f"{DUMP_BYTES >> 20} MB)")
     ap.add_argument("--probe", default=None, choices=["batch", "stream"], help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm sizes its work by timing, its output is not fixed)")
     if args.probe:
         return probe_main(args.probe)
     global PROBE_VARIANT
@@ -485,7 +509,8 @@ def main():
     def ptrs(a):
         return (ctypes.c_void_p * a.shape[0])(*[a[c].ctypes.data for c in range(a.shape[0])])
 
-    def time_steps(step, steps, stream, with_clocks, frames):
+    def time_steps(step, steps, stream, with_clocks, frames, after_timed=None):
+        """`after_timed` runs right after the last timed step, before anything else touches the output"""
         for _ in range(warm):
             step()
         barrier()
@@ -504,6 +529,8 @@ def main():
             ev[i][1].record(stream)
         barrier()
         t_w1 = time.perf_counter()
+        if after_timed:
+            after_timed()
         ms_per_step = allmax(sum(a.elapsed_time(b) for a, b in ev)) / steps
         if with_clocks:
             # K short steps give nvidia-smi (>= 20 ms per sample) almost nothing to see: EVERY rank keeps the very
@@ -585,7 +612,15 @@ def main():
         }
 
     # ------------------------------------------------------------------------------------------
-    def run_single_or_partition(wl, T, steps, with_e2e, with_clocks, with_parity, tag):
+    def sampled_output(y_dev, C, T, block, keep=None):
+        """the dump_blocks() sample of a (C, T * block) device output; blocks outside [keep) are zeroed"""
+        blocks = dump_blocks(T, C, block)
+        y = y_dev.view(C, T, block).index_select(1, torch.from_numpy(blocks).to(y_dev.device))
+        if keep is not None:
+            y[:, (blocks < keep[0]) | (blocks >= keep[1])] = 0.0
+        return y
+
+    def run_single_or_partition(wl, T, steps, with_e2e, with_clocks, with_parity, tag, want_dump=False):
         """world == 1: the unsharded engine.  world > 1: partition-range shards (+ slot exchange / NCCL reduce)."""
         from oracle import refcheck as rc
         C, block = wl["C"], wl["block"]
@@ -632,8 +667,14 @@ def main():
         def step_device():
             eng.process_device(x_dev.data_ptr(), n, y_dev.data_ptr(), n, n, sync=False)
 
+        dump = {}
+
+        def keep_output():      # partition-range shards: shard 0 holds the whole output
+            if want_dump:
+                dump["y"] = sampled_output(y_dev, C, T, block).cpu().numpy()
+
         launches0 = eng.launch_count
-        ms_per_step, value, clocks = time_steps(step_device, steps, stream, with_clocks, n)
+        ms_per_step, value, clocks = time_steps(step_device, steps, stream, with_clocks, n, keep_output)
         launches = eng.launch_count - launches0
         roof = sweep_roofline(eng, lambda: eng.process_device(x_dev.data_ptr(), n, y_dev.data_ptr(), n, n, sync=True),
                               C, block, Ploc, T, eng.stages(), n)
@@ -696,7 +737,7 @@ def main():
             barrier()
         res = {
             "value": value, "ms_per_step": ms_per_step, "launches": int(allsum(launches)), "clocks": clocks, "e2e": e2e,
-            "parity": parity, "roofline": roof,
+            "parity": parity, "roofline": roof, "dump": dump,
             "config": {"workload": wl["desc"], "channels": C, "ir_taps": eng.ir_len(0), "block": block, "partitions": P,
                        "blocks_per_step": T, "frames_per_step": n, "launch_groups_per_step": groups,
                        "parallelism": mgpu_path if world == 1 else f"x{world}: {mgpu_path} ({Ploc} partitions on rank 0)",
@@ -708,7 +749,7 @@ def main():
         return res
 
     # ------------------------------------------------------------------------------------------
-    def run_time_sliced(wl, T, steps, with_e2e, with_clocks, with_parity, tag):
+    def run_time_sliced(wl, T, steps, with_e2e, with_clocks, with_parity, tag, want_dump=False):
         """world > 1, batch >> IR: every GPU holds the whole convolver and produces one time slice of the batch."""
         from oracle import refcheck as rc
         C, block = wl["C"], wl["block"]
@@ -749,8 +790,16 @@ def main():
         def step_device():
             eng.process_device_sliced(x_dev.data_ptr(), n, y_dev.data_ptr(), n, n, rank, world, sync=False)
 
+        dump = {}
+
+        def keep_output():      # every rank holds its own slice [a, b) of the output: sum the masked samples
+            if want_dump:
+                y = sampled_output(y_dev, C, T, block, keep=(a, b))
+                dist.all_reduce(y)
+                dump["y"] = y.cpu().numpy()
+
         launches0 = eng.launch_count
-        ms_per_step, value, clocks = time_steps(step_device, steps, stream, with_clocks, n)
+        ms_per_step, value, clocks = time_steps(step_device, steps, stream, with_clocks, n, keep_output)
         launches = eng.launch_count - launches0
         roof = sweep_roofline(eng, lambda: eng.process_device_sliced(x_dev.data_ptr(), n, y_dev.data_ptr(), n, n, rank, world, sync=True),
                               C, block, P, b - a, eng.stages(), (b - a) * block)
@@ -821,7 +870,7 @@ def main():
             barrier()
         res = {
             "value": value, "ms_per_step": ms_per_step, "launches": int(allsum(launches)), "clocks": clocks, "e2e": e2e,
-            "parity": parity, "roofline": roof,
+            "parity": parity, "roofline": roof, "dump": dump,
             "config": {"workload": wl["desc"], "channels": C, "ir_taps": eng.ir_len(0), "block": block, "partitions": P,
                        "blocks_per_step": T, "frames_per_step": n, "launch_groups_per_step": 1,
                        "parallelism": f"x{world}: time-slice sharding — every GPU holds the whole convolver ({P} partitions) and convolves "
@@ -837,7 +886,8 @@ def main():
     T = args.blocks or (T_METRIC if args.workload == "metric" else (7104 * 512 // wl["block"] if "tail" in wl else 7104))
     sliced = world > 1 and args.metric_shards == "time" and "tail" not in wl and args.workload != "ir120"
     runner = run_time_sliced if sliced else run_single_or_partition
-    main_res = runner(wl, T, args.steps, with_e2e=not args.no_e2e, with_clocks=True, with_parity=not args.no_parity, tag="m")
+    main_res = runner(wl, T, args.steps, with_e2e=not args.no_e2e, with_clocks=True, with_parity=not args.no_parity, tag="m",
+                      want_dump=bool(args.dump_outputs))
     extra = None
     if not args.no_ir120 and args.workload == "metric":
         try:
@@ -1002,6 +1052,10 @@ def main():
             line["realtime_process"] = realtime
         if offline:
             line["offline_block8192"] = offline
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in main_res["dump"].items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line))
         for name, p in (("metric", main_res["parity"]), ("ir120", (extra or {}).get("parity"))):
             if p and not p.get("ok", True):

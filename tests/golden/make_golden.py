@@ -1,12 +1,21 @@
 """Generates tests/golden/*.npz from the UNMODIFIED reference (oracle/_ref).
 
-Run in the build container (needs /root/reference or a prebuilt oracle/_ref):
+Run where oracle/_ref can be built (the original project's sources, see oracle/Makefile):
     python -m tests.golden.make_golden
 Each fixture stores the case parameters, a checksum of the regenerated inputs and the
 reference output `out`; `run_case` re-creates the inputs and drives any implementation that
 offers the reference surface (init/process/clear), so the same function checks the C oracle
 (tests/test_oracle.py) and the CUDA path (tests/test_gpu_parity.py).
+
+Three more fixtures, under reference/, pin the C restatements in oracle/ to the reference where the
+tests used to need the compiled reference at test time:
+  ref_selftest_cases.npz   reference output of the 58 self-test cases (tests/refcases.py)
+  ref_apply_decay.npz      the STFT decay driven through the reference's own AudioFFT
+  ref_filter.npz           the reference Filter: coefficients and the SHA-256 of every output
+Long outputs are stored as a sample (`sample_points`) plus the peak of the whole output, so the
+tests keep their tolerance relative to the full output's peak.
 """
+import hashlib
 import os
 import sys
 import zlib
@@ -14,6 +23,7 @@ import zlib
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+REFERENCE = os.path.join(HERE, "reference")
 ROOT = os.path.dirname(os.path.dirname(HERE))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -90,14 +100,110 @@ def run_case(spec, impl="oracle"):
     return y
 
 
+def sample_points(n: int, k: int = 256) -> np.ndarray:
+    """Indices of the stored sample of an n-sample output: all of them when n <= k, else the first and last k/4 and
+    k/2 seeded random ones in between (sorted)."""
+    if n <= k:
+        return np.arange(n, dtype=np.int32)
+    q = k // 4
+    mid = np.random.default_rng(n).choice(np.arange(q, n - q), k - 2 * q, replace=False)
+    return np.sort(np.concatenate([np.arange(q), mid, np.arange(n - q, n)])).astype(np.int32)
+
+
+def selftest_key(kind: str, case) -> str:
+    return kind[0] + "-" + "-".join(map(str, case))
+
+
+def selftest_run(kind: str, case, impl: str) -> np.ndarray:
+    """One case of the reference self-test (ramps, glibc rand() chunking) through the oracle or the reference."""
+    x, h = rc.ramp(case[0]), rc.ramp(case[1])
+    total = case[0] + case[1] - 1
+    chunks = rc.chunk_schedule(total, case[2], case[3], rc.GlibcRand(1))
+    if kind == "uniform":
+        conv = orc.RefUniform() if impl == "ref" else orc.OracleUniform()
+        assert conv.init(case[4], h)
+    else:
+        conv = orc.RefTwoStage() if impl == "ref" else orc.OracleTwoStage()
+        assert conv.init(case[4], case[5], h)
+    return rc.drive(conv, x, total, chunks)
+
+
+DECAY_LENGTHS = (30000, 5000, 4096, 1025, 100)
+
+
+def decay_luts():
+    return (np.ones(2049), np.linspace(1.0, 0.7, 2049), np.linspace(0.8, 1.05, 2049))
+
+
+FILTER_RATES = (44100.0, 48000.0, 96000.0)
+FILTER_FREQS = (20.0, 55.5, 300.0, 1234.0, 8000.0, 19999.0, 30000.0)
+
+
+def filter_input() -> np.ndarray:
+    return np.random.default_rng(3).standard_normal(6000).astype(np.float32)
+
+
+def filter_q(slope: int) -> float:
+    return 0.0765 if slope == 2 else 0.2929
+
+
+def sha256_u8(a: np.ndarray) -> np.ndarray:
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), dtype=np.uint8)
+
+
+def make_ref_selftest_cases() -> dict:
+    out = {}
+    for kind, cases in (("uniform", rc.UNIFORM_CASES), ("twostage", rc.TWOSTAGE_CASES)):
+        for case in cases:
+            y = selftest_run(kind, case, "ref")
+            idx = sample_points(y.size)
+            k = selftest_key(kind, case)
+            out[k + "_idx"], out[k + "_out"], out[k + "_peak"] = idx, y[idx], np.float64(np.max(np.abs(y)))
+    return out
+
+
+def make_ref_apply_decay() -> dict:
+    out = {}
+    for n in DECAY_LENGTHS:
+        h = orc.synth_ir(n)
+        for j, lut in enumerate(decay_luts()):
+            y = orc.ref_apply_decay(h, lut, 48000.0)
+            idx = sample_points(y.size)
+            k = f"n{n}_lut{j}"
+            out[k + "_idx"], out[k + "_out"], out[k + "_peak"] = idx, y[idx], np.float64(np.max(np.abs(y)))
+    return out
+
+
+def make_ref_filter() -> dict:
+    """coeff[rate, freq]; sha256 / sample[rate, freq, slope, mode] of the filtered filter_input()"""
+    x = filter_input()
+    idx = sample_points(x.size, 64)
+    coeff = np.zeros((len(FILTER_RATES), len(FILTER_FREQS)))
+    sha = np.zeros((len(FILTER_RATES), len(FILTER_FREQS), 3, 3, 32), np.uint8)
+    sample = np.zeros((len(FILTER_RATES), len(FILTER_FREQS), 3, 3, idx.size), np.float32)
+    for i, sr in enumerate(FILTER_RATES):
+        for j, fr in enumerate(FILTER_FREQS):
+            coeff[i, j] = orc.filter_coeff(fr, sr, ref=True)
+            for slope in range(3):
+                for mode in range(3):
+                    y = orc.RefFilter(slope, mode, sr, fr, filter_q(slope)).run(x)
+                    sha[i, j, slope, mode] = sha256_u8(y)
+                    sample[i, j, slope, mode] = y[idx]
+    return dict(coeff=coeff, sha256=sha, idx=idx, sample=sample)
+
+
 def main():
-    assert orc.ref_available(), "needs oracle/_ref (the compiled reference)"
+    assert orc.ref_available() and orc.ref_filter_available(), "needs oracle/_ref (the compiled reference)"
     for name, spec in CASES.items():
         x, h = _signals(spec)
         spec = dict(spec, in_crc=zlib.crc32(x.tobytes()), ir_crc=zlib.crc32(h.tobytes()))
         out = run_case(spec, impl="ref")
         np.savez_compressed(os.path.join(HERE, name + ".npz"), out=out, **spec)
         print(f"{name}: {out.size} samples, peak {np.abs(out).max():.4g}")
+    for name, make in (("ref_selftest_cases", make_ref_selftest_cases), ("ref_apply_decay", make_ref_apply_decay),
+                       ("ref_filter", make_ref_filter)):
+        np.savez_compressed(os.path.join(REFERENCE, name + ".npz"), **make())
+        print(f"{name}: written")
 
 
 if __name__ == "__main__":

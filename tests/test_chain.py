@@ -1,11 +1,15 @@
 """SURVEY 8f-4 + the rest of 8f-1: the send / wet chain of processBlock on the device (b200conv_chain_process) against
-its oracle (oracle/chain_oracle.c), which is PINNED by the reference's own Filter.cpp compiled into oracle/_ref."""
+its oracle (oracle/chain_oracle.c), which is PINNED by the reference's own Filter.cpp compiled into oracle/_ref (its
+outputs are stored in tests/golden/reference/ref_filter.npz)."""
+import os
+
 import numpy as np
 import pytest
 
 from oracle import oracle as orc
 from reevr_b200.convolver import Engine
 from tests.backends import lib  # noqa: F401
+from tests.golden import make_golden as mg
 
 TOL = 1e-5
 
@@ -14,18 +18,17 @@ def peak_err(y, ref):
     return float(np.max(np.abs(y - ref)) / max(np.max(np.abs(ref)), 1e-30))
 
 
-@pytest.mark.skipif(not orc.ref_filter_available(), reason="oracle/_ref/libreffilter.so not built and /root/reference absent")
 def test_filter_restatement_is_bit_identical_to_the_reference_filter():
-    x = np.random.default_rng(3).standard_normal(6000).astype(np.float32)
-    for sr in (44100.0, 48000.0, 96000.0):
-        for fr in (20.0, 55.5, 300.0, 1234.0, 8000.0, 19999.0, 30000.0):
-            assert orc.filter_coeff(fr, sr) == orc.filter_coeff(fr, sr, ref=True)
+    g = np.load(os.path.join(mg.REFERENCE, "ref_filter.npz"))
+    x = mg.filter_input()
+    for i, sr in enumerate(mg.FILTER_RATES):
+        for j, fr in enumerate(mg.FILTER_FREQS):
+            assert orc.filter_coeff(fr, sr) == g["coeff"][i, j]
             for slope in (0, 1, 2):
                 for mode in (0, 1, 2):
-                    q = 0.0765 if slope == 2 else 0.2929
-                    a = orc.OracleFilter(slope, mode, sr, fr, q).run(x)
-                    b = orc.RefFilter(slope, mode, sr, fr, q).run(x)
-                    assert np.array_equal(a, b), (sr, fr, slope, mode)
+                    a = orc.OracleFilter(slope, mode, sr, fr, mg.filter_q(slope)).run(x)
+                    assert np.array_equal(a[g["idx"]], g["sample"][i, j, slope, mode]), (sr, fr, slope, mode)
+                    assert np.array_equal(mg.sha256_u8(a), g["sha256"][i, j, slope, mode]), (sr, fr, slope, mode)
 
 
 def _reference_chain(cfg, irs, head, tail, L, R, ysend, yrev, chunks):

@@ -1,7 +1,8 @@
 """Pins the CPU oracle (oracle/partconv_oracle.c) — runs without a GPU.
 
 1. the reference's own 58 known-answer cases (naive-convolution truth, reference tolerance);
-2. the unmodified reference compiled here (oracle/_ref), same chunking, tight tolerance;
+2. the unmodified reference's output for the same cases and chunking, tight tolerance
+   (tests/golden/reference/ref_selftest_cases.npz, generated from oracle/_ref);
 3. the committed golden fixtures (tests/golden/*.npz, generated from oracle/_ref).
 """
 import glob
@@ -12,6 +13,7 @@ import pytest
 
 from oracle import oracle as orc
 from tests import refcases as rc
+from tests.golden import make_golden as mg
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -21,40 +23,31 @@ def _peak_err(a, b):
     return d / max(np.max(np.abs(b.astype(np.float64))), 1e-30)
 
 
+def _reference_err(fixture, key, y):
+    """peak error of y against the reference's stored sample of the same output, relative to its whole peak"""
+    g = np.load(os.path.join(mg.REFERENCE, fixture + ".npz"))
+    idx = g[key + "_idx"]
+    assert idx[-1] == y.size - 1                   # the stored sample always ends on the last sample
+    d = np.max(np.abs(y[idx].astype(np.float64) - g[key + "_out"].astype(np.float64)))
+    return d / max(float(g[key + "_peak"]), 1e-30)
+
+
 @pytest.mark.parametrize("case", rc.UNIFORM_CASES, ids=lambda c: "u-" + "-".join(map(str, c)))
 def test_uniform_selftest_cases(case):
-    n_in, n_ir, bmin, bmax, block = case
-    x, h = rc.ramp(n_in), rc.ramp(n_ir)
-    total = n_in + n_ir - 1
-    chunks = rc.chunk_schedule(total, bmin, bmax, rc.GlibcRand(1))
-    conv = orc.OracleUniform()
-    assert conv.init(block, h)
-    y = rc.drive(conv, x, total, chunks)
-    truth = orc.naive_convolve(x, h)
+    n_in, n_ir = case[:2]
+    y = mg.selftest_run("uniform", case, "oracle")
+    truth = orc.naive_convolve(rc.ramp(n_in), rc.ramp(n_ir))
     assert rc.reference_selftest_ok(y, truth, n_ir)
-    if orc.ref_available():
-        ref = orc.RefUniform()
-        assert ref.init(block, h)
-        yr = rc.drive(ref, x, total, chunks)
-        assert _peak_err(y, yr) <= 1e-6
+    assert _reference_err("ref_selftest_cases", mg.selftest_key("uniform", case), y) <= 1e-6
 
 
 @pytest.mark.parametrize("case", rc.TWOSTAGE_CASES, ids=lambda c: "t-" + "-".join(map(str, c)))
 def test_twostage_selftest_cases(case):
-    n_in, n_ir, bmin, bmax, head, tail = case
-    x, h = rc.ramp(n_in), rc.ramp(n_ir)
-    total = n_in + n_ir - 1
-    chunks = rc.chunk_schedule(total, bmin, bmax, rc.GlibcRand(1))
-    conv = orc.OracleTwoStage()
-    assert conv.init(head, tail, h)
-    y = rc.drive(conv, x, total, chunks)
-    truth = orc.naive_convolve(x, h)
+    n_in, n_ir = case[:2]
+    y = mg.selftest_run("twostage", case, "oracle")
+    truth = orc.naive_convolve(rc.ramp(n_in), rc.ramp(n_ir))
     assert rc.reference_selftest_ok(y, truth, n_ir)
-    if orc.ref_available():
-        ref = orc.RefTwoStage()
-        assert ref.init(head, tail, h)
-        yr = rc.drive(ref, x, total, chunks)
-        assert _peak_err(y, yr) <= 1e-6
+    assert _reference_err("ref_selftest_cases", mg.selftest_key("twostage", case), y) <= 1e-6
 
 
 def test_error_conventions():
@@ -143,13 +136,12 @@ def test_apply_decay_restatement_properties():
     assert np.sum(got[-8000:] ** 2) < 0.2 * np.sum(h[-8000:] ** 2)      # the tail really decays faster
 
 
-@pytest.mark.skipif(not orc.ref_available(), reason="oracle/_ref not built and /root/reference absent")
 def test_apply_decay_restatement_pinned_by_the_reference_fft():
     """oc_apply_decay (Impulse::applyDecay restated, own FFT) against the same STFT loop driven through the reference's
-    compiled audiofft::AudioFFT (oracle/ref_shim.cpp::ref_stft_decay): the (f3) oracle is no longer unpinned."""
-    for n in (30000, 5000, 4096, 1025, 100):
+    compiled audiofft::AudioFFT (oracle/ref_shim.cpp::ref_stft_decay, stored in tests/golden/reference/ref_apply_decay.npz):
+    the (f3) oracle is no longer unpinned."""
+    for n in mg.DECAY_LENGTHS:
         h = orc.synth_ir(n)
-        for lut in (np.ones(2049), np.linspace(1.0, 0.7, 2049), np.linspace(0.8, 1.05, 2049)):
+        for j, lut in enumerate(mg.decay_luts()):
             a = orc.apply_decay(h, lut, 48000.0)
-            b = orc.ref_apply_decay(h, lut, 48000.0)
-            assert np.max(np.abs(a - b)) <= 1e-6 * max(np.max(np.abs(b)), 1e-30)
+            assert _reference_err("ref_apply_decay", f"n{n}_lut{j}", a) <= 1e-6, (n, j)
