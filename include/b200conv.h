@@ -42,7 +42,8 @@ typedef struct b200conv_config {
   int shard_rank;        /* partition-range shard owned by this handle (multi-GPU), 0 <= rank < n   */
   int shard_count;       /* number of shards (1 = unsharded)                                        */
   int cmac_variant;      /* 0 = auto; >0 selects a specific CMAC kernel variant (tuning/bench):     */
-                         /* 22 packed-FMA batched, 40 tensor cores (tcgen05), 100..108 streaming    */
+                         /* 22 packed-FMA batched, 40 tensor cores (tcgen05), 50..52 FFT along the */
+                         /* block axis, 100..108 streaming                                         */
 } b200conv_config;
 
 /* Lifetime ------------------------------------------------------------------------------- */

@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libb200conv.so")
 SOURCES = ["engine.cu", "irshape.cu"]
-DEPS = ["engine.cu", "irshape.cu", "kernels.cuh", "kernels_stream.cuh", "kernels_fft512.cuh", "kernels_rt.cuh", "kernels_chain.cuh", "kernels_tc.cuh",
+DEPS = ["engine.cu", "irshape.cu", "kernels.cuh", "kernels_stream.cuh", "kernels_fft512.cuh", "kernels_rt.cuh", "kernels_chain.cuh", "kernels_tc.cuh", "kernels_tfft.cuh",
         os.path.join("..", "..", "include", "b200conv.h")]
 
 NVCC_FLAGS = [

@@ -43,6 +43,7 @@
 #include "kernels_fft512.cuh"
 #include "kernels_rt.cuh"
 #include "kernels_chain.cuh"
+#include "kernels_tfft.cuh"
 #if !defined(PC_EMULATE)
 #include "kernels_tc.cuh"
 #endif
@@ -180,6 +181,17 @@ struct b200conv {
   int* tc_err_dev = nullptr;
   bool tc_attr_set = false;
   bool tc_alloc_failed = false;      // the scratch did not fit once: stay on the FFMA sweep
+  // FFT sweep along the block axis (kernels_tfft.cuh): filter spectra of one stage's H, twiddles of the length-N transform
+  bool opt_tfft = std::getenv("B200CONV_NO_TFFT") == nullptr;
+  float2* tfft_Hf = nullptr;
+  size_t tfft_Hf_bytes = 0;
+  const void* tfft_Hf_for = nullptr;   // H the spectra were built from (+ its geometry)
+  int tfft_Hf_P = 0, tfft_Hf_B = 0, tfft_Hf_C = 0, tfft_Hf_N = 0;
+  float2* tfft_tw = nullptr;
+  size_t tfft_tw_bytes = 0;
+  int tfft_tw_N = 0;
+  bool tfft_attr_set[3] = {false, false, false};
+  bool tfft_alloc_failed = false;    // the spectra did not fit once: stay on the other sweeps
   int last_variant = 0;              // sweep form the last launch_cmac resolved to (b200conv_last_sweep_variant)
   // slot exchange (fused multi-GPU path), stage 0 of a single-stage handle
   bool p2p_on = false;
@@ -280,6 +292,9 @@ void free_all(b200conv* h) {
   h->tc_A = h->tc_Xt = h->tc_Yt = nullptr; h->tc_A_for = nullptr; h->tc_A_bytes = h->tc_Xt_bytes = h->tc_Yt_bytes = 0;
   if (h->tc_err) cudaFreeHost(h->tc_err);
   h->tc_err = h->tc_err_dev = nullptr; h->tc_alloc_failed = false;
+  cudaFree(h->tfft_Hf); cudaFree(h->tfft_tw);
+  h->tfft_Hf = h->tfft_tw = nullptr; h->tfft_Hf_for = nullptr; h->tfft_Hf_bytes = h->tfft_tw_bytes = 0; h->tfft_tw_N = 0;
+  h->tfft_alloc_failed = false;
   cudaFree(h->c_io); cudaFree(h->c_conv_in); cudaFree(h->c_filt); cudaFree(h->c_state); cudaFree(h->c_ring);
   if (h->c_hpin) cudaFreeHost(h->c_hpin);
   h->c_hpin = h->c_hpin_dev = nullptr;
@@ -326,6 +341,26 @@ void timing_collect(b200conv* h) {
     else if (h->ev_pool[i].kind == kKindFft) h->t_fft += ms;
     else h->t_ifft += ms;
   }
+}
+
+// twiddle table of the M-point transforms (layout: kernels.cuh tw_pass_offset), computed in double
+std::vector<float2> fft_twiddles(int M) {
+  std::vector<float2> tw(pc::tw_table_len(M));
+  for (int k = 0; k <= M / 2; ++k) {                       // split twiddles exp(-2*pi*i*k/(2M))
+    const double a = -2.0 * M_PI * (double)k / (2.0 * (double)M);
+    tw[k] = make_float2((float)std::cos(a), (float)std::sin(a));
+  }
+  for (int p = 1; p < M;) {                                // pass twiddles exp(-2*pi*i*r*k/(p*R))
+    const int R = pc::pass_radix(M, p);
+    const int off = pc::tw_pass_offset(M, p);
+    for (int r = 1; r < R; ++r)
+      for (int k = 0; k < p; ++k) {
+        const double a = -2.0 * M_PI * (double)r * (double)k / ((double)p * (double)R);
+        tw[off + (r - 1) * p + k] = make_float2((float)std::cos(a), (float)std::sin(a));
+      }
+    p *= R;
+  }
+  return tw;
 }
 
 // ---- kernel launchers ----------------------------------------------------------------------
@@ -660,6 +695,8 @@ int launch_cmac_stream_tma(b200conv* h, const pc::CmacParams& P, int C, int stag
 
 // ---- tensor-core sweep (kernels_tc.cuh) -------------------------------------------------------------------------
 constexpr int kTcMinBlocks = 4096;      // below that a 128-segment tile is mostly padding: the FFMA sweep is faster
+constexpr int kTfftMinBins = 256;       // automatic FFT sweep along the block axis: the range it was measured in
+constexpr int kTfftMinParts = 256;
 
 // can this sweep run on the tensor cores?  (geometry only; the scratch is allocated by launch_cmac_tc)
 bool tc_eligible(const b200conv* h, const pc::CmacParams& P, int C) {
@@ -674,17 +711,17 @@ bool tc_eligible(const b200conv* h, const pc::CmacParams& P, int C) {
 #endif
 }
 
-#if !defined(PC_EMULATE)
-// grow-only device scratch; a failed allocation is not an error of the call (the caller falls back to the FFMA sweep)
-bool tc_reserve(b200conv* h, float** buf, size_t* have, size_t need) {
+// grow-only device scratch; a failed allocation is not an error of the call (the caller falls back to another
+// sweep and sets *failed so that later launch groups do not try again)
+template <class T>
+bool grow_reserve(T** buf, size_t* have, size_t need, bool* failed) {
   if (*have >= need) return true;
   cudaFree(*buf);
   *buf = nullptr; *have = 0;
-  if (cudaMalloc(buf, need) != cudaSuccess) { cudaGetLastError(); *buf = nullptr; h->tc_alloc_failed = true; return false; }
+  if (cudaMalloc((void**)buf, need) != cudaSuccess) { cudaGetLastError(); *buf = nullptr; *failed = true; return false; }
   *have = need;
   return true;
 }
-#endif
 
 // returns 1 when the scratch could not be allocated (nothing launched), 0 on success, < 0 on error
 int launch_cmac_tc(b200conv* h, const pc::CmacParams& P, int C) {
@@ -702,13 +739,13 @@ int launch_cmac_tc(b200conv* h, const pc::CmacParams& P, int C) {
   }
   if (*reinterpret_cast<volatile int*>(h->tc_err) != 0)
     return fail(h, B200CONV_ECUDA, "tensor-core sweep: a pipeline barrier timed out (code " + std::to_string(*h->tc_err) + ")");
-  if (!tc_reserve(h, &h->tc_Xt, &h->tc_Xt_bytes, lines * 4 * (size_t)g.Lt * sizeof(float))) return 1;
-  if (!tc_reserve(h, &h->tc_Yt, &h->tc_Yt_bytes, lines * 4 * (size_t)g.Lty * sizeof(float))) return 1;
+  if (!grow_reserve(&h->tc_Xt, &h->tc_Xt_bytes, lines * 4 * (size_t)g.Lt * sizeof(float), &h->tc_alloc_failed)) return 1;
+  if (!grow_reserve(&h->tc_Yt, &h->tc_Yt_bytes, lines * 4 * (size_t)g.Lty * sizeof(float), &h->tc_alloc_failed)) return 1;
   const size_t a_bytes = lines * (size_t)g.nchunk * 2 * tc::kATileBytes;
   const bool a_stale = h->tc_A_for != P.H || h->tc_A_P != P.Ppad || h->tc_A_B != P.B || h->tc_A_C != C || h->tc_A_bytes < a_bytes;
   if (a_stale) {
     h->tc_A_for = nullptr;
-    if (!tc_reserve(h, &h->tc_A, &h->tc_A_bytes, a_bytes)) return 1;
+    if (!grow_reserve(&h->tc_A, &h->tc_A_bytes, a_bytes, &h->tc_alloc_failed)) return 1;
   }
   if (!h->tc_attr_set) {
     CU_CHECK(h, cudaFuncSetAttribute(tc::k_tc_sweep, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemBytes));
@@ -736,9 +773,95 @@ int launch_cmac_tc(b200conv* h, const pc::CmacParams& P, int C) {
 #endif
 }
 
+// ---- FFT sweep along the block axis (kernels_tfft.cuh) ---------------------------------------------------------
+// cmac_variant 50: N = 4096, G = 4 (the automatic choice); 51: N = 2048, G = 4; 52: N = 2048, G = 8
+struct TfftShape { int N, G; };
+inline TfftShape tfft_shape(int variant) {
+  return variant == 51 ? TfftShape{2048, 4} : variant == 52 ? TfftShape{2048, 8} : TfftShape{4096, 4};
+}
+
+bool tfft_eligible(const pc::CmacParams& P, int C, int variant) {
+  const TfftShape s = tfft_shape(variant);
+  if (P.xg > 0 || P.Ppad < 1 || P.nblocks < 1 || P.B % s.G != 0) return false;
+  if (P.Ppad - 1 > pc::tfft_qmax(s.N)) return false;
+  const pc::TfftGeom g = pc::tfft_geom(s.N, P.Ppad, P.nblocks);
+  return (unsigned long long)C * (P.B / s.G) * (unsigned long long)g.nseg < (1ull << 31);
+}
+
+template <int N, int G>
+void tfft_launch_t(b200conv* h, const pc::TfftBuildParams* bp, const pc::TfftParams& wp, int C, int ntiles) {
+#if defined(PC_EMULATE)
+  if (bp) pc::emu_tfft_build_h<N, G>(C, *bp);
+  pc::emu_tfft_sweep<N, G>(C, wp);
+  (void)h; (void)ntiles;
+#else
+  constexpr size_t smem = pc::tfft_smem_bytes(N, G);
+  constexpr int nt = pc::tfft_threads(N, G);
+  if (bp) pc::k_tfft_build_h<N, G><<<dim3(bp->B / G, C), nt, smem, h->s_launch>>>(*bp);
+  pc::k_tfft_sweep<N, G><<<ntiles, nt, smem, h->s_launch>>>(wp);
+#endif
+}
+
+// returns 1 when the filter spectra could not be allocated (nothing launched), 0 on success, < 0 on error
+int launch_cmac_tfft(b200conv* h, const pc::CmacParams& P, int C, int variant) {
+  const TfftShape s = tfft_shape(variant);
+  const size_t hf_bytes = (size_t)C * P.B * s.N * sizeof(float2);
+  const bool stale = h->tfft_Hf_for != P.H || h->tfft_Hf_P != P.Ppad || h->tfft_Hf_B != P.B || h->tfft_Hf_C != C ||
+                     h->tfft_Hf_N != s.N || h->tfft_Hf_bytes < hf_bytes;
+  if (stale) {
+    h->tfft_Hf_for = nullptr;
+    if (!grow_reserve(&h->tfft_Hf, &h->tfft_Hf_bytes, hf_bytes, &h->tfft_alloc_failed)) return 1;
+  }
+  if (h->tfft_tw_N != s.N) {
+    const std::vector<float2> tw = fft_twiddles(s.N);
+    h->tfft_tw_N = 0;
+    if (!grow_reserve(&h->tfft_tw, &h->tfft_tw_bytes, tw.size() * sizeof(float2), &h->tfft_alloc_failed)) return 1;
+    CU_CHECK(h, cudaMemcpyAsync(h->tfft_tw, tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice, h->s_launch));
+    CU_CHECK(h, cudaStreamSynchronize(h->s_launch));
+    h->tfft_tw_N = s.N;
+  }
+#if !defined(PC_EMULATE)
+  const int vi = variant - 50;
+  if (!h->tfft_attr_set[vi]) {
+    if (variant == 51) {
+      CU_CHECK(h, cudaFuncSetAttribute(pc::k_tfft_sweep<2048, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pc::tfft_smem_bytes(2048, 4)));
+      CU_CHECK(h, cudaFuncSetAttribute(pc::k_tfft_build_h<2048, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pc::tfft_smem_bytes(2048, 4)));
+    } else if (variant == 52) {
+      CU_CHECK(h, cudaFuncSetAttribute(pc::k_tfft_sweep<2048, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pc::tfft_smem_bytes(2048, 8)));
+      CU_CHECK(h, cudaFuncSetAttribute(pc::k_tfft_build_h<2048, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pc::tfft_smem_bytes(2048, 8)));
+    } else {
+      CU_CHECK(h, cudaFuncSetAttribute(pc::k_tfft_sweep<4096, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pc::tfft_smem_bytes(4096, 4)));
+      CU_CHECK(h, cudaFuncSetAttribute(pc::k_tfft_build_h<4096, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pc::tfft_smem_bytes(4096, 4)));
+    }
+    h->tfft_attr_set[vi] = true;
+  }
+#endif
+  const pc::TfftGeom g = pc::tfft_geom(s.N, P.Ppad, P.nblocks);
+  pc::TfftBuildParams bp{P.H, P.h_cstride, h->tfft_Hf, h->tfft_tw, P.B, P.Ppad};
+  pc::TfftParams wp{P.X, P.x_cstride, P.xrow0, std::max<long long>(0, P.xrow0 - (P.Ppad - 1)), P.xrow0 + P.nblocks,
+                    h->tfft_Hf, P.Y, P.y_cstride, P.y_rstride, P.yrow0, h->tfft_tw, P.B, P.nblocks, g.Q, g.Lo, g.nseg};
+  const int ntiles = C * (P.B / s.G) * g.nseg;
+  int id = timing_begin(h, kKindCmac);
+  switch (variant) {     // once per IR (and stage) the filter spectra first, then the sweep
+    case 51: tfft_launch_t<2048, 4>(h, stale ? &bp : nullptr, wp, C, ntiles); break;
+    case 52: tfft_launch_t<2048, 8>(h, stale ? &bp : nullptr, wp, C, ntiles); break;
+    default: tfft_launch_t<4096, 4>(h, stale ? &bp : nullptr, wp, C, ntiles); break;
+  }
+  timing_end(h, id);
+  if (stale) {
+    h->tfft_Hf_for = P.H; h->tfft_Hf_P = P.Ppad; h->tfft_Hf_B = P.B; h->tfft_Hf_C = C; h->tfft_Hf_N = s.N;
+    h->launches++;
+  }
+  h->launches++;
+  CU_CHECK(h, cudaGetLastError());
+  return 0;
+}
+
 // P.Ppad enters as the number of real (unpadded) partition rows of this shard
 int launch_cmac(b200conv* h, const pc::CmacParams& P, int C) {
   int variant = h->cfg.cmac_variant;
+  if (P.xg > 0 && variant >= 50 && variant <= 52)
+    return fail(h, B200CONV_EINVAL, "FFT sweep along the block axis: the slot exchange is not supported");
   if (P.xg > 0) variant = (P.nblocks >= 64) ? 22 : 26;     // slot exchange: only the packed-FMA sweeps carry the exchange epilogue
   if (variant == 0) {
     // streaming sweep for real-time calls; packed-FMA batched sweep otherwise (TT = 16 when the
@@ -752,10 +875,24 @@ int launch_cmac(b200conv* h, const pc::CmacParams& P, int C) {
     }
     else if (P.nblocks <= kStreamNBS && P.B >= 64 && P.Ppad >= 1) variant = 101;
     else if (P.nblocks <= kStreamNBS && P.B >= 2 && P.Ppad >= 1) variant = 100;
+    // FFT along the block axis where it measured faster than the tensor-core sweep (profiles/r03_*)
+    else if (h->opt_tfft && !h->tfft_alloc_failed && P.nblocks >= kTcMinBlocks && P.B >= kTfftMinBins &&
+             P.Ppad >= kTfftMinParts && tfft_eligible(P, C, 50)) variant = 50;
     else if (h->opt_tc && !h->tc_alloc_failed && P.nblocks >= kTcMinBlocks && tc_eligible(h, P, C)) variant = 40;
     else variant = (P.nblocks >= 64) ? 22 : 26;
   }
   h->last_variant = variant;
+  if (variant >= 50 && variant <= 52) {
+    if (!tfft_eligible(P, C, variant))
+      return fail(h, B200CONV_EINVAL, "FFT sweep along the block axis: unsupported shape (needs B a multiple of the bin group, "
+                                      "P - 1 <= 3/4 of the transform length, no slot exchange)");
+    const int rc = launch_cmac_tfft(h, P, C, variant);
+    if (rc <= 0) return rc;
+    if (h->cfg.cmac_variant == variant) return fail(h, B200CONV_ENOMEM, "FFT sweep along the block axis: filter spectra allocation failed");
+    // not enough device memory for the spectra
+    variant = (h->opt_tc && !h->tc_alloc_failed && P.nblocks >= kTcMinBlocks && tc_eligible(h, P, C)) ? 40 : (P.nblocks >= 64) ? 22 : 26;
+    h->last_variant = variant;
+  }
   if (variant == 40) {                         // tcgen05 3xTF32 block-Toeplitz sweep
     if (!tc_eligible(h, P, C)) return fail(h, B200CONV_EINVAL, "tensor-core sweep: unsupported shape (needs B % 32 == 0, at most 961 partitions, no slot exchange)");
     const int rc = launch_cmac_tc(h, P, C);
@@ -853,23 +990,8 @@ int build_stage(b200conv* h, Stage& s, const float* const* ir, const std::vector
   s.Prows = round_up(std::max(s.P, 1), kPadP) + kDPre;
   s.hist = s.p_begin + round_up(std::max(s.P, 1), kPadP) + kDPre;
 
-  // twiddle table (layout: kernels.cuh tw_pass_offset), computed in double
-  const int N = pc::tw_table_len(B);
-  std::vector<float2> tw(N);
-  for (int k = 0; k <= B / 2; ++k) {                       // split twiddles exp(-2*pi*i*k/(2B))
-    const double a = -2.0 * M_PI * (double)k / (2.0 * (double)B);
-    tw[k] = make_float2((float)std::cos(a), (float)std::sin(a));
-  }
-  for (int p = 1; p < B;) {                                // pass twiddles exp(-2*pi*i*r*k/(p*R))
-    const int R = pc::pass_radix(B, p);
-    const int off = pc::tw_pass_offset(B, p);
-    for (int r = 1; r < R; ++r)
-      for (int k = 0; k < p; ++k) {
-        const double a = -2.0 * M_PI * (double)r * (double)k / ((double)p * (double)R);
-        tw[off + (r - 1) * p + k] = make_float2((float)std::cos(a), (float)std::sin(a));
-      }
-    p *= R;
-  }
+  const std::vector<float2> tw = fft_twiddles(B);
+  const int N = (int)tw.size();
   CU_CHECK(h, cudaMalloc(&s.tw, N * sizeof(float2)));
   CU_CHECK(h, cudaMemcpyAsync(s.tw, tw.data(), N * sizeof(float2), cudaMemcpyHostToDevice, h->s_main));
   std::vector<float2> t512;
@@ -2507,6 +2629,7 @@ int b200conv_set_option(b200conv_t* h, const char* name, int value) {
   else if (n == "slice_keep_tail") h->opt_slice_tail = value != 0;
   else if (n == "stream_alternate") h->opt_stream_alt = value != 0;
   else if (n == "tc") h->opt_tc = value != 0;
+  else if (n == "tfft") h->opt_tfft = value != 0;
   else return fail(h, B200CONV_EINVAL, "unknown option");
   return B200CONV_OK;
 }
